@@ -2,7 +2,7 @@
 """bench.py -- policy steps/sec of the VIMA policy forward pass on B200 (contract: see the task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3|cfg2|cfg3x|cfg5]
-                    [--precision f16f8] [--ragged] [--graph]
+                    [--precision f16f8] [--ragged] [--graph] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one policy step for every episode of the batch, exactly as scripts/example.py chains the policy's
@@ -25,6 +25,10 @@ Workloads (BASELINE.json configs / SURVEY.md 8(d) rows):
               bench.py runs the same `--impl reference` code in a subprocess, so the two numbers share one code path.
 `gpu_eager` : the same unmodified reference in PyTorch eager on the SAME GPU (fp32, and TF32-allowed), full batch, with the
               rel-L2 between its outputs and ours on identical inputs and weights.
+`--dump-outputs DIR`: what the last device-timed step returned on rank 0 -- normalised and raw action logits [B, 700] in
+              ActionDecoder key order (logits, logits_raw), the action indices per key (mode.<key>, as float64) and the next
+              action token (action_token) -- as DIR/<name>.npy.  Inputs and weights are seeded, so two builds run with the same
+              arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -66,7 +70,12 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-eager", action="store_true")
     ap.add_argument("--no-incremental", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, for output-by-output comparison of two builds")
+    args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs at least one timed step")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -232,6 +241,37 @@ def raw_logits(dists) -> torch.Tensor:
 
 def norm_logits(dists) -> torch.Tensor:
     return torch.cat([d.logits for k in dists for d in dists[k]._dists], dim=-1).reshape(-1, 700)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(dists, modes, nxt) -> dict:
+    """What one policy step hands its caller, as host arrays: name -> (float32/float64 array, episode axis)."""
+    out = {"logits": (norm_logits(dists).float().cpu().numpy(), 0), "logits_raw": (raw_logits(dists).float().cpu().numpy(), 0),
+           "action_token": (nxt.float().cpu().numpy(), 1)}
+    for k, v in modes.items():  # action indices, exact in float64
+        out[f"mode.{k}"] = (v.cpu().numpy().astype("float64"), 1)
+    return out
+
+
+def dump_outputs(path: str, outputs: dict) -> None:
+    """Writes path/<name>.npy.  Above DUMP_LIMIT_BYTES in all, every array keeps the same fixed, seeded sample of episodes
+    (listed in episodes.npy), so that two runs with the same arguments still compare element for element."""
+    import numpy as np
+
+    total = sum(a.nbytes for a, _ in outputs.values())
+    budget = DUMP_LIMIT_BYTES - 4096 * (len(outputs) + 1)  # .npy headers
+    if total > budget:
+        a0, ax0 = next(iter(outputs.values()))
+        n_ep = a0.shape[ax0]
+        per_episode = total / n_ep + 8  # + its float64 entry in episodes.npy
+        keep = np.sort(np.random.default_rng(0).choice(n_ep, max(1, int(budget // per_episode)), replace=False))
+        outputs = {k: (np.take(a, keep, axis=ax), ax) for k, (a, ax) in outputs.items()}
+        outputs["episodes"] = (keep.astype("float64"), 0)
+    os.makedirs(path, exist_ok=True)
+    for k, (a, _) in outputs.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -598,11 +638,13 @@ def run_ours(args):
         torch.cuda.nvtx.range_push("timed")
         e0.record()
         for _ in range(args.steps):
-            run_step(new_obs_dev)
+            last = run_step(new_obs_dev)
         e1.record()
         barrier()
         torch.cuda.nvtx.range_pop()
         gt.on = False
+        if args.dump_outputs and rank == 0:  # now: the replays below overwrite the graph's static outputs
+            dump_outputs(args.dump_outputs, step_outputs(*last))
         ms_total = e0.elapsed_time(e1)
         launches = ctx.launches - launches0
         if use_graph:

@@ -6,7 +6,7 @@ import torch
 
 from oracle import detgen, synth, vima_oracle as O
 from oracle.state_dict_spec import flamingo_state_dict_spec
-from tests.util import assert_close, golden_pick, load_golden, rel_l2
+from tests.util import assert_close, golden_pick, load_golden, reference_state_dict, rel_l2
 
 NAME = "flamingo_small"
 
@@ -72,19 +72,13 @@ def test_flamingo_state_dict_contract():
         assert tuple(v.shape) == tuple(spec[k]), k
 
 
-@pytest.mark.reference
 def test_flamingo_spec_matches_reference():
-    import sys
-
-    from oracle.ref_shim import load_reference
-
-    load_reference()
     cfg = synth.FLAMINGO_CFGS["flamingo_tiny"]
-    sd = sys.modules["vima.policy"].VIMAFlamingoPolicy(**cfg).state_dict()
+    sd = dict(reference_state_dict("VIMAFlamingoPolicy/flamingo_tiny", cfg))
     spec = flamingo_state_dict_spec(**cfg)
     assert sorted(sd.keys()) == sorted(spec.keys())
-    for k, v in sd.items():
-        assert tuple(v.shape) == tuple(spec[k]), k
+    for k, shape in sd.items():
+        assert shape == tuple(spec[k]), k
 
 
 @pytest.mark.gpu

@@ -5,7 +5,7 @@ import torch
 
 from oracle import detgen, synth, vima_oracle as O
 from oracle.state_dict_spec import gato_state_dict_spec
-from tests.util import assert_close, golden_pick, load_golden, rel_l2
+from tests.util import assert_close, golden_pick, load_golden, reference_state_dict, rel_l2
 
 NAME = "gato_small"
 
@@ -57,17 +57,13 @@ def test_gato_state_dict_contract():
     pol.load_state_dict(sd2, strict=True)
 
 
-@pytest.mark.reference
 def test_gato_spec_matches_reference():
-    from oracle.ref_shim import load_reference
-
-    ref = load_reference()
     cfg = synth.GATO_CFGS["gato_tiny"]
-    sd = ref.VIMAGatoPolicy(**cfg).state_dict()
+    sd = dict(reference_state_dict("VIMAGatoPolicy/gato_tiny", cfg))
     spec = gato_state_dict_spec(**cfg)
     assert sorted(sd.keys()) == sorted(spec.keys())
-    for k, v in sd.items():
-        assert tuple(v.shape) == tuple(spec[k]), k
+    for k, shape in sd.items():
+        assert shape == tuple(spec[k]), k
 
 
 @pytest.mark.gpu

@@ -6,7 +6,7 @@ import torch
 
 from oracle import detgen, synth, vima_oracle as O
 from oracle.state_dict_spec import gpt_state_dict_spec
-from tests.util import assert_close, golden_pick, load_golden, rel_l2
+from tests.util import assert_close, golden_pick, load_golden, reference_state_dict, rel_l2
 
 NAME = "gpt_small"
 
@@ -65,19 +65,13 @@ def test_gpt_state_dict_contract():
     subprocess.run([sys.executable, "-c", code], cwd=root, check=True, env={**os.environ, "PYTHONPATH": root})
 
 
-@pytest.mark.reference
 def test_gpt_spec_matches_reference():
-    import sys
-
-    from oracle.ref_shim import load_reference
-
-    load_reference()
     cfg = synth.GATO_CFGS["gato_tiny"]
-    sd = sys.modules["vima.policy"].VIMAGPTPolicy(**cfg).state_dict()
+    sd = dict(reference_state_dict("VIMAGPTPolicy/gato_tiny", cfg))
     spec = gpt_state_dict_spec(**cfg)
     assert sorted(sd.keys()) == sorted(spec.keys())
-    for k, v in sd.items():
-        assert tuple(v.shape) == tuple(spec[k]), k
+    for k, shape in sd.items():
+        assert shape == tuple(spec[k]), k
 
 
 @pytest.mark.gpu

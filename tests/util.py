@@ -14,6 +14,16 @@ def load_golden(case: str) -> dict:
     return dict(np.load(os.path.join(GOLDEN_DIR, f"{case}.npz")))
 
 
+def reference_state_dict(name: str, cfg: dict) -> list:
+    """[(key, shape)] in order of the reference policy's state dict, recorded by tests/golden/make_state_dict_golden.py."""
+    import json
+
+    with open(os.path.join(GOLDEN_DIR, "reference_state_dicts.json")) as fh:
+        entry = json.load(fh)[name]
+    assert entry["cfg"] == dict(cfg), (name, entry["cfg"], cfg)  # the recording is of this configuration
+    return [(k, tuple(shape)) for k, shape in entry["state_dict"]]
+
+
 def golden_pick(g: dict, name: str, actual: torch.Tensor):
     """Returns (expected, actual) numpy arrays laid out alike; undoes the strided storage of large tensors."""
     a = actual.detach().cpu()
